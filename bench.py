@@ -4,7 +4,7 @@ iterations per second on the 4-camera x 400-frame
 LENSMODEL_SPLINED_STEREOGRAPHIC_order=3_Nx=30_Ny=20_fov_x_deg=170 synthetic
 calibration (BASELINE config 3).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3] [--dump-outputs DIR]
 
 A "step" is one complete solve of the problem from the same seed. Prints ONE JSON
 line (rank 0). See DESIGN.md "Measurement" for what every field means.
@@ -167,6 +167,19 @@ def solve_config5(world, rank, local_rank, max_iterations):
     return out
 
 
+def dump_outputs(directory, arrays):
+    """Writes what the timed path returned in its last step as DIR/<name>.npy (float64), so that two builds can be
+    compared output for output: the inputs come from fixed seeds and are the same from run to run. Outputs the
+    workload does not have (no discrete points, say) come back empty and are not written; scalars become 1-vectors."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if a is None:
+            continue
+        a = np.atleast_1d(np.asarray(a, dtype=np.float64))
+        if a.size:
+            np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def measure_fp64_peak():
     """cuBLAS DGEMM throughput, the denominator for the fp64-tensor roofline (not in MEASURED_PEAKS.json)."""
     import torch
@@ -202,6 +215,10 @@ def main():
                          "measurement); the numbers printed are not bench values")
     ap.add_argument("--max-iterations", type=int, default=300,
                     help="cap on trust-region iterations per solve (300 = the reference's; smaller only for profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the solution of the last one (b_packed, x, the unpacked state and "
+                         "the observation weights; with --gpus > 1 the gathered state), its rms and outlier count as "
+                         "DIR/<name>.npy in float64")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -280,6 +297,16 @@ def main():
         infos.append(one_step())
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # read back before anything else runs on P; sharded, the full-size solution arrays are gathered from every rank
+        if shard is None:
+            sol = P.download(into_inputs=False)
+        else:
+            from mrcal_b200 import distributed
+            sol = distributed.gather_solution(P, shard)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dict(sol, rms_reproj_error__pixels=infos[-1]["rms_reproj_error__pixels"],
+                                                 Noutliers_board=infos[-1]["Noutliers_board"]))
 
     ms = np.array([i["ms_total"] for i in infos])
     its = np.array([i["Niterations"] for i in infos])

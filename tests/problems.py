@@ -3,9 +3,13 @@
 Every case is rebuilt from mrcal_b200.synthetic.make_problem() with a fixed seed,
 so the inputs exist wherever the repo does; tests/golden/callback_cases.npz holds
 what the COMPILED REFERENCE computed for them (tests/golden/make_golden.py)."""
+import os
+
 import numpy as np
 
 from mrcal_b200 import synthetic
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 SPL3 = "LENSMODEL_SPLINED_STEREOGRAPHIC_order=3_Nx=11_Ny=8_fov_x_deg=150"
 SPL2 = "LENSMODEL_SPLINED_STEREOGRAPHIC_order=2_Nx=12_Ny=9_fov_x_deg=150"
@@ -120,6 +124,11 @@ def golden_cases():
         tri_only=True)
     add("tri_stereographic_unity", "LENSMODEL_STEREOGRAPHIC", 3, 3, _sel(False, False, True, True, False, unity=True), Ntri=4)
     return cases
+
+
+def oracle_golden(group):
+    """What the compiled reference computed for the inputs of one test module (tests/golden/make_oracle_golden.py)."""
+    return np.load(os.path.join(GOLDEN, f"oracle_{group}.npz"))
 
 
 def layout_numbers(P):

@@ -16,7 +16,8 @@ import problems
 # mrcal_b200.cameramodel is the CLASS (as mrcal.cameramodel is); the module holds the helpers too
 cm = importlib.import_module("mrcal_b200.cameramodel")
 
-REFDATA = "/root/reference/test/data"
+# the reference's own model files (its test/data), stored as data fixtures
+MODELS = os.path.join(problems.GOLDEN, "cameramodels")
 
 
 def test_roundtrip_explicit_model():
@@ -46,11 +47,15 @@ def test_roundtrip_explicit_model():
         cm.cameramodel(intrinsics=("LENSMODEL_OPENCV8", intr[:8]), imagersize=(10, 10))
 
 
-def test_inverse_pose_matches_reference(ref):
-    rng = np.random.default_rng(0)
-    for _ in range(5):
-        rt = rng.normal(size=6)
-        assert np.allclose(cm.invert_rt(rt), ref.invert_rt(rt), atol=1e-12)
+def inverse_pose_inputs():
+    return np.random.default_rng(0).normal(size=(5, 6))
+
+
+def test_inverse_pose_matches_reference():
+    gold = problems.oracle_golden("cameramodel")
+    assert np.array_equal(gold["rt"], inverse_pose_inputs())
+    for rt, inverted_ref in zip(gold["rt"], gold["inverted"]):
+        assert np.allclose(cm.invert_rt(rt), inverted_ref, atol=1e-12)
     assert np.allclose(cm.invert_rt(np.array((0., 0., 0., 1., 2., 3.))), (0., 0., 0., -1., -2., -3.))
 
 
@@ -99,9 +104,8 @@ def test_legacy_names_and_errors():
         cm.cameramodel(text.replace("'imagersize'", "'icam_intrinsics': 0, 'imagersize'"))
 
 
-@pytest.mark.skipif(not os.path.isdir(REFDATA), reason="the reference tree is not mounted here")
 def test_reads_the_reference_files():
-    files = sorted(glob.glob(os.path.join(REFDATA, "*.cameramodel")))
+    files = sorted(glob.glob(os.path.join(MODELS, "*.cameramodel")))
     assert files
     for path in files:
         m = cm.cameramodel(path)

@@ -49,7 +49,7 @@ def test_A_Jt_J_At(Nx):
         mrcal_b200._A_Jt_J_At(A, Jp, Ji, Jx)
 
 
-def test_on_a_calibration_jacobian(ref):
+def test_on_a_calibration_jacobian():
     """The shapes the uncertainty code uses: J of a calibration problem, A = 2 x Nstate, board rows only."""
     import mrcal_b200
     from mrcal_b200 import synthetic

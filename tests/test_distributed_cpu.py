@@ -1,7 +1,10 @@
 """The N>1 path on CPU: two processes over gloo. Checks the host-side sharding
 (mrcal_b200/distributed.py) and, with the compiled reference as the cost function, the
 ALGORITHM of the sharded solve: the per-rank Schur-reduced normal equations, summed with
-an all-reduce, equal the reduced normal equations of the whole problem (SURVEY.md 8e)."""
+an all-reduce, equal the reduced normal equations of the whole problem (SURVEY.md 8e).
+The reduced systems of the reference's Jacobians are stored under tests/golden/ for the
+shards shard_inputs() makes today; a digest of each shard's inputs ties them together."""
+import hashlib
 import os
 import sys
 
@@ -12,6 +15,27 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+WORLD = 2
+
+
+def problem():
+    from mrcal_b200 import synthetic
+    kw, _ = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV4", Ncameras=3, Nframes=9, W=5, H=4, seed=4,
+                                   pixel_noise=0.2, Npoints=10, Npoints_fixed=2, which="some")
+    return kw
+
+
+def digest(kw):
+    h = hashlib.sha256()
+    for k in sorted(kw):
+        v = kw[k]
+        h.update(k.encode())
+        if isinstance(v, np.ndarray):
+            h.update(f"{v.dtype.str}{v.shape}".encode())
+            h.update(np.ascontiguousarray(v).tobytes())
+        else:
+            h.update(repr(v).encode())
+    return h.hexdigest()
 
 
 def _reduced(J, x, e0, e1):
@@ -33,11 +57,13 @@ def _worker(rank, world, port, q):
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
         import mrcal_b200
-        from mrcal_b200 import distributed, synthetic
-        from oracle import ref
-        kw, _ = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV4", Ncameras=3, Nframes=9, W=5, H=4, seed=4,
-                                       pixel_noise=0.2, Npoints=10, Npoints_fixed=2, which="some")
+        import problems
+        from mrcal_b200 import distributed
+        gold = problems.oracle_golden("distributed")
+        kw = problem()
         kw_local, shard = distributed.shard_inputs(kw, rank, world)
+        # the stored reduced systems are those of exactly these shards
+        assert digest(kw_local) == str(gold[f"rank{rank}/digest"])
         # 1. the local slice is a valid problem by the reference's own rules (mrcal-pywrap.c:976-1244)
         I = mrcal_b200.api._Inputs(dict(kw_local))
         # 2. shards tile the frames and the observations
@@ -50,29 +76,20 @@ def _worker(rank, world, port, q):
         assert ts[:, 3].sum() == kw["observations_point"].shape[0]
         assert ts[:, 4].sum() == kw["rt_ref_frame"].shape[0]
         assert ts[:, 5].sum() == kw["points"].shape[0] - 2
-        # 3. the shared unknowns are laid out identically on every rank
-        Pl = ref.Problem(kw_local)
-        n_shared = Pl.num_states() - Pl.num_states_of("frames") - Pl.num_states_of("points")
+        # 3. the shared unknowns are laid out identically on every rank, by the reference and by the product
+        n_shared = int(gold[f"rank{rank}/n_shared"])
+        assert n_shared == (mrcal_b200.num_states(**kw_local) - mrcal_b200.num_states_frames(**kw_local)
+                            - mrcal_b200.num_states_points(**kw_local))
         tt = torch.tensor([n_shared]); tts = [torch.zeros_like(tt) for _ in range(world)]
         dist.all_gather(tts, tt)
         assert all(int(v) == n_shared for v in tts)
         # 4. sum over ranks of the locally reduced systems == the reduced system of the whole problem.
-        #    Regularization rows are replicated: only rank 0 counts them
-        b, x, J = Pl.callback()
-        nreg = Pl.num_measurements_of("regularization")
-        if rank != 0 and nreg:
-            J = J[:-nreg]
-            x = x[:-nreg]
-        e0 = Pl.state_index("frames", 0)
-        e1 = e0 + Pl.num_states_of("frames") + Pl.num_states_of("points")
-        S, g, _, _ = _reduced(J, x, e0, e1)
-        St, gt = torch.from_numpy(S.copy()), torch.from_numpy(g.copy())
+        #    Regularization rows are replicated: only rank 0 counts them (_reduced() of the reference's J)
+        St, gt = torch.from_numpy(gold[f"rank{rank}/S"].copy()), torch.from_numpy(gold[f"rank{rank}/g"].copy())
         dist.all_reduce(St)
         dist.all_reduce(gt)
-        Pg = ref.Problem(kw)
-        bg, xg, Jg = Pg.callback()
-        e0g = Pg.state_index("frames", 0)
-        Sg, gg, scaleA, scaleg = _reduced(Jg, xg, e0g, e0g + Pg.num_states_of("frames") + Pg.num_states_of("points"))
+        Sg, gg = gold["global/S"], gold["global/g"]
+        scaleA, scaleg = gold["global/scales"]
         assert np.abs(St.numpy() - Sg).max() <= 1e-9 * scaleA
         assert np.abs(gt.numpy() - gg).max() <= 1e-9 * scaleg
         q.put((rank, "ok"))
@@ -83,8 +100,8 @@ def _worker(rank, world, port, q):
         dist.destroy_process_group()
 
 
-def test_sharding_two_ranks_gloo(ref):
-    world = 2
+def test_sharding_two_ranks_gloo():
+    world = WORLD
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29500 + (os.getpid() % 400)

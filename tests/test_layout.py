@@ -1,5 +1,5 @@
 """State/measurement layout, lens-model descriptions and pack/unpack of the C-ABI
-library versus the compiled reference (oracle/_ref) and the stored golden numbers.
+library versus what the compiled reference (oracle/_ref) computed, stored under tests/golden/.
 Pure integer / scale logic: runs without a GPU. Model: the exact identities the
 reference checks in test/test-basic-calibration.py:168-232."""
 import ctypes as C
@@ -18,49 +18,55 @@ LENSMODELS = ("LENSMODEL_PINHOLE", "LENSMODEL_STEREOGRAPHIC", "LENSMODEL_LONLAT"
               problems.SPL3, problems.SPL2, problems.SPL3_BIG)
 
 
-def test_lensmodel_parsing_matches_reference(ref):
-    for name in LENSMODELS:
-        a = ref.lensmodel_from_name(name)
+BAD_LENSMODELS = ("LENSMODEL_OPENCV7", "LENSMODEL_SPLINED_STEREOGRAPHIC", "LENSMODEL_SPLINED_STEREOGRAPHIC_order=3",
+                  "LENSMODEL_SPLINED_STEREOGRAPHIC_order=3_Nx=30_Ny=20_fov_x_deg=170x", "LENSMODEL_CAHVORE", "",
+                  "LENSMODEL_OPENCV8_")
+SPLINED = (problems.SPL3, problems.SPL2, problems.SPL3_BIG)
+PRECOMPUTED_LENSMODELS = SPLINED + ("LENSMODEL_OPENCV8",)
+TRIANGULATED_CASES = ("tri_pinhole_only", "tri_opencv4_boards_points", "tri_stereographic_unity")
+
+
+@pytest.fixture(scope="module")
+def gold():
+    return problems.oracle_golden("layout")
+
+
+def test_lensmodel_parsing_matches_reference(gold):
+    for i, name in enumerate(LENSMODELS):
+        assert str(gold[f"lensmodel{i}/name"]) == name
+        a = gold[f"lensmodel{i}/struct"].tobytes()
         b = mrcal_b200.api._lensmodel(name)
-        assert bytes(a)[:4] == bytes(b)[:4] and bytes(a)[8:] == bytes(b)[8:], name
-        assert ref.lensmodel_num_params(name) == mrcal_b200.lensmodel_num_params(name)
+        assert a[:4] == bytes(b)[:4] and a[8:] == bytes(b)[8:], name
+        assert int(gold[f"lensmodel{i}/num_params"]) == mrcal_b200.lensmodel_num_params(name)
         buf = C.create_string_buffer(256)
         assert _capi.lib.mrcal_lensmodel_name(buf, 256, C.byref(b))
-        buf2 = C.create_string_buffer(256)
-        ref.lib().mrcal_lensmodel_name(buf2, 256, C.byref(a))
-        assert buf.value == buf2.value
-    for bad in ("LENSMODEL_OPENCV7", "LENSMODEL_SPLINED_STEREOGRAPHIC", "LENSMODEL_SPLINED_STEREOGRAPHIC_order=3",
-                "LENSMODEL_SPLINED_STEREOGRAPHIC_order=3_Nx=30_Ny=20_fov_x_deg=170x", "LENSMODEL_CAHVORE", "",
-                "LENSMODEL_OPENCV8_"):
-        ra, rb = ref.Lensmodel(), _capi.Lensmodel()
-        ok_ref = ref.lib().mrcal_lensmodel_from_name(C.byref(ra), bad.encode())
+        assert buf.value.decode() == str(gold[f"lensmodel{i}/written_name"])
+    for i, bad in enumerate(BAD_LENSMODELS):
+        ok_ref, type_ref, type_from_name_ref = gold[f"bad{i}"]
+        rb = _capi.Lensmodel()
         ok = _capi.lib.mrcal_lensmodel_from_name(C.byref(rb), bad.encode())
-        assert bool(ok_ref) == bool(ok) and ra.type == rb.type, bad
+        assert bool(ok_ref) == bool(ok) and type_ref == rb.type, bad
         with pytest.raises(RuntimeError):
             mrcal_b200.lensmodel_num_params(bad)
-        assert ref.lib().mrcal_lensmodel_type_from_name(bad.encode()) == \
-            _capi.lib.mrcal_lensmodel_type_from_name(bad.encode())
+        assert type_from_name_ref == _capi.lib.mrcal_lensmodel_type_from_name(bad.encode())
 
 
-def test_precomputed_lensmodel_data_matches_reference(ref):
+def test_precomputed_lensmodel_data_matches_reference(gold):
     class Pre(C.Structure):
         _fields_ = [("ready", C.c_bool), ("segments_per_u", C.c_double)]
-    for name in (problems.SPL3, problems.SPL2, problems.SPL3_BIG, "LENSMODEL_OPENCV8"):
-        a, b = Pre(), Pre()
-        ref.lib()._mrcal_precompute_lensmodel_data(C.byref(a), C.byref(ref.lensmodel_from_name(name)))
+    for i, name in enumerate(PRECOMPUTED_LENSMODELS):
+        ready_ref, segments_per_u_ref = gold[f"precomputed{i}"]
+        b = Pre()
         _capi.lib._mrcal_precompute_lensmodel_data(C.byref(b), C.byref(mrcal_b200.api._lensmodel(name)))
-        assert a.ready and b.ready
+        assert ready_ref and b.ready
         if "SPLINED" in name:
-            assert a.segments_per_u == b.segments_per_u and a.segments_per_u > 0
+            assert segments_per_u_ref == b.segments_per_u and segments_per_u_ref > 0
 
 
-def test_knots_match_reference(ref):
-    for name in (problems.SPL3, problems.SPL2, problems.SPL3_BIG):
+def test_knots_match_reference(gold):
+    for i, name in enumerate(SPLINED):
         ux, uy = mrcal_b200.knots_for_splined_models(name)
-        lm = ref.lensmodel_from_name(name)
-        rx, ry = np.zeros_like(ux), np.zeros_like(uy)
-        ref.lib().mrcal_knots_for_splined_models(rx.ctypes.data_as(C.c_void_p), ry.ctypes.data_as(C.c_void_p), C.byref(lm))
-        assert np.array_equal(ux, rx) and np.array_equal(uy, ry)
+        assert np.array_equal(ux, gold[f"knots{i}/x"]) and np.array_equal(uy, gold[f"knots{i}/y"])
 
 
 def _layout_numbers_product(kw):
@@ -87,14 +93,13 @@ def test_layout_matches_stored_reference_numbers():
         assert _layout_numbers_product(kw) == list(g[f"{name}__layout"]), name
 
 
-def test_layout_matches_compiled_reference_on_a_grid(ref):
-    """All 2^7 selections x lens models x shapes, every layout function."""
+def layout_grid():
+    """(what, optimization_inputs): all 2^7 selections x lens models x shapes, with zero-valued arrays."""
     rng = np.random.default_rng(0)
     shapes = [(1, 0, 3, 0, 0, 3, 0), (2, 1, 4, 0, 0, 6, 0), (3, 2, 2, 5, 2, 4, 9), (2, 2, 0, 4, 0, 0, 6), (4, 3, 5, 3, 3, 11, 5)]
     names = [n for n in _capi.SELECTION_BITS if n != "do_apply_outlier_rejection"]
-    nchecked = 0
     for lm in ("LENSMODEL_PINHOLE", "LENSMODEL_OPENCV8", "LENSMODEL_OPENCV12", "LENSMODEL_CAHVOR", problems.SPL3, problems.SPL2):
-        Nintr = ref.lensmodel_num_params(lm)
+        Nintr = mrcal_b200.lensmodel_num_params(lm)
         for (Nci, Nce, Nf, Np, Npf, Nob, Nop) in shapes:
             idx_b = np.zeros((Nob, 3), np.int32)
             if Nob:
@@ -112,11 +117,17 @@ def test_layout_matches_compiled_reference_on_a_grid(ref):
                         observations_point=np.zeros((Nop, 3)), indices_point_camintrinsics_camextrinsics=idx_p,
                         Npoints_fixed=Npf, calobject_warp=np.zeros(2), calibration_object_spacing=0.1)
             for bits in itertools.product((False, True), repeat=len(names)):
-                kw = dict(base, **dict(zip(names, bits)))
-                P = ref.Problem(kw)
-                assert _layout_numbers_product(kw) == problems.layout_numbers(P), (lm, Nci, Nce, Nf, Np, Npf, Nob, Nop, bits)
-                nchecked += 1
-    assert nchecked > 3000
+                yield (lm, Nci, Nce, Nf, Np, Npf, Nob, Nop, bits), dict(base, **dict(zip(names, bits)))
+
+
+def test_layout_matches_compiled_reference_on_a_grid(gold):
+    """All 2^7 selections x lens models x shapes, every layout function."""
+    grid = gold["grid"]
+    nchecked = 0
+    for k, (what, kw) in enumerate(layout_grid()):
+        assert _layout_numbers_product(kw) == list(grid[k]), what
+        nchecked += 1
+    assert nchecked == len(grid) and nchecked > 3000
 
 
 def test_explicit_counts_interface():
@@ -142,18 +153,18 @@ def test_explicit_counts_interface():
         m.num_states(Ncameras_intrinsics=1)   # lensmodel is required
 
 
-def test_pack_unpack_matches_reference(ref):
+def test_pack_unpack_matches_reference(gold):
     rng = np.random.default_rng(1)
     for name, kw in problems.golden_cases():
-        P = ref.Problem(kw)
-        n = P.num_states()
-        b = rng.normal(size=(3, n))
-        mine, theirs = b.copy(), b.copy()
+        # the reference's pack divides by the scale of each state and its unpack multiplies by it
+        scale = gold[f"{name}/state_scale"]
+        b = rng.normal(size=(3, len(scale)))
+        mine = b.copy()
         mrcal_b200.pack_state(mine, **kw)
-        P.pack_vector(theirs)
+        theirs = b / scale
         assert np.array_equal(mine, theirs), name
         mrcal_b200.unpack_state(mine, **kw)
-        P.unpack_vector(theirs)
+        theirs = theirs * scale
         assert np.array_equal(mine, theirs), name
         assert np.allclose(mine, b, rtol=1e-15, atol=0)
     with pytest.raises(RuntimeError):
@@ -166,15 +177,15 @@ def test_corresponding_icam_extrinsics():
     assert mrcal_b200.corresponding_icam_extrinsics(2, **kw) == 1
 
 
-def test_triangulated_layout_and_validation(ref):
+def test_triangulated_layout_and_validation(gold):
     """The layout functions with triangulated points need the SETS only (no rays, no GPU): compare with the
     compiled reference, and check the wrapper's complaints (mrcal-pywrap.c:1207-1240, 1406-1440)."""
     cases = dict(problems.golden_cases())
-    for name in ("tri_pinhole_only", "tri_opencv4_boards_points", "tri_stereographic_unity"):
+    for name in TRIANGULATED_CASES:
         kw = cases[name]
-        P = ref.Problem(kw)
-        assert mrcal_b200.num_measurements(**kw) == P.num_measurements()
-        assert mrcal_b200.api._Inputs(dict(kw), for_layout_only=True).num_j_nonzero() == P.num_j_nonzero()
+        num_measurements_ref, num_j_nonzero_ref = gold[f"{name}/num_measurements"]
+        assert mrcal_b200.num_measurements(**kw) == num_measurements_ref
+        assert mrcal_b200.api._Inputs(dict(kw), for_layout_only=True).num_j_nonzero() == num_j_nonzero_ref
         Ntri = mrcal_b200.num_measurements_points_triangulated(**kw)
         idx = kw["indices_point_triangulated_camintrinsics_camextrinsics"]
         assert Ntri == sum(n * (n - 1) // 2 for n in np.bincount(idx[:, 0]))

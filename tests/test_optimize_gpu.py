@@ -1,13 +1,12 @@
 """mrcal_b200.optimize() (through the reference-named C-ABI entry mrcal_optimize())
 against the CPU restatement of the reference's solve: oracle/dogleg_np.py driving
-the compiled reference's cost function (oracle/_ref).
+the compiled reference's cost function (oracle/_ref). What that restatement returned is stored under
+tests/golden/ by tests/golden/make_oracle_golden.py.
 
 Gates (BASELINE.md): |b_packed - b_ref|_inf <= 1e-5, |rms - rms_ref| <= 1e-7 px,
 norm2_x relative 1e-9, same outlier set. The iterate sequence is not pinned by the
 reference (oracle/dogleg_np.py header); on these well-conditioned problems the two
 implementations take the same number of steps, which is asserted too."""
-import copy
-
 import numpy as np
 import pytest
 
@@ -29,11 +28,96 @@ def clone(kw):
     return {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in kw.items()}
 
 
-def run_both(kw):
-    from oracle import dogleg_np
-    kw_gpu, kw_cpu = clone(kw), clone(kw)
-    r_cpu = dogleg_np.optimize(kw_cpu)
+# the caller's arrays the solution is written into
+STATE_ARRAYS = ("intrinsics", "rt_cam_ref", "rt_ref_frame", "points", "calobject_warp")
+RESTATEMENT = [
+    ("LENSMODEL_OPENCV8", 2, 8),
+    ("LENSMODEL_OPENCV4", 3, 6),
+    ("LENSMODEL_PINHOLE", 1, 5),
+    ("LENSMODEL_STEREOGRAPHIC", 2, 5),
+    ("LENSMODEL_CAHVOR", 2, 8),
+    ("LENSMODEL_CAHVORE_linearity=0.37", 2, 8),
+    (SPL3_COVERED, 2, 40),
+    (SPL2_COVERED, 2, 40),
+]
+SELECTIONS = [
+    dict(do_optimize_intrinsics_core=False, do_optimize_intrinsics_distortions=False, do_optimize_extrinsics=False,
+         do_optimize_frames=True, do_optimize_calobject_warp=False),    # frames only: nothing shared
+    dict(do_optimize_intrinsics_core=True, do_optimize_intrinsics_distortions=True, do_optimize_extrinsics=False,
+         do_optimize_frames=False, do_optimize_calobject_warp=False),   # intrinsics only: nothing eliminated
+    dict(do_optimize_intrinsics_core=False, do_optimize_intrinsics_distortions=False, do_optimize_extrinsics=True,
+         do_optimize_frames=True, do_optimize_calobject_warp=True),
+]
+TRIANGULATED = ["tri_pinhole_unity_only", "tri_opencv4_boards_points", "tri_stereographic_unity"]
+TIGHT = dict(update_threshold=1e-24, max_iterations=2000)
+
+
+def _restatement(lensmodel, Ncameras, Nframes):
+    kw, truth = synthetic.make_problem(lensmodel=lensmodel, Ncameras=Ncameras, Nframes=Nframes, W=6, H=5, seed=2,
+                                       pixel_noise=0.2)
+    return kw
+
+
+def _with_points():
+    kw, truth = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV4", Ncameras=3, Nframes=8, W=6, H=5, seed=4,
+                                       pixel_noise=0.2, Npoints=12, Npoints_fixed=3, which="some")
+    return kw
+
+
+def _selection(i):
+    kw, truth = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV8", Ncameras=2, Nframes=6, W=6, H=5, seed=5,
+                                       pixel_noise=0.2, perturb=0.3)
+    kw.update(SELECTIONS[i])
+    return kw
+
+
+def _triangulated(name):
+    kw = clone(dict(problems.golden_cases())[name])
+    kw["do_apply_outlier_rejection"] = False
+    return kw
+
+
+def _outlier_rejection():
+    kw, truth = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV4", Ncameras=2, Nframes=12, W=8, H=7, seed=6,
+                                       pixel_noise=0.3)
+    rng = np.random.default_rng(0)
+    flat = kw["observations_board"].reshape(-1, 3)
+    bad = rng.choice(flat.shape[0], 15, replace=False)
+    flat[bad, :2] += rng.normal(0, 30., (15, 2))          # gross outliers
+    flat[rng.choice(flat.shape[0], 5, replace=False), 2] = -1.   # pre-marked outliers are respected
+    kw["do_apply_outlier_rejection"] = True
+    return kw
+
+
+def cases():
+    """{case: optimization_inputs} of the solves compared with the CPU restatement"""
+    out = {f"restatement/{lm}": _restatement(lm, Nc, Nf) for lm, Nc, Nf in RESTATEMENT}
+    out["points"] = _with_points()
+    out.update({f"selection/{i}": _selection(i) for i in range(len(SELECTIONS))})
+    out.update({f"triangulated/{name}": _triangulated(name) for name in TRIANGULATED})
+    out["outlier_rejection"] = _outlier_rejection()
+    return out
+
+
+def tight_cases():
+    return {lm: _restatement(lm, 2, 40) for lm in (SPL3_COVERED, SPL2_COVERED)}
+
+
+@pytest.fixture(scope="module")
+def gold():
+    return problems.oracle_golden("optimize")
+
+
+def run_both(gold, case, kw):
+    """This library's solve of kw, the arrays it wrote the solution into, and what the CPU restatement returned."""
+    kw_gpu = clone(kw)
     r_gpu = mrcal_b200.optimize(**kw_gpu)
+    rms, norm2_x = gold[f"{case}/scalars"]
+    Noutliers_board, passes = gold[f"{case}/counts"]
+    r_cpu = dict(b_packed=gold[f"{case}/b_packed"], rms_reproj_error__pixels=rms, norm2_x=norm2_x,
+                 Noutliers_board=int(Noutliers_board), passes=int(passes),
+                 state={k: gold[f"{case}/{k}"] for k in STATE_ARRAYS if f"{case}/{k}" in gold},
+                 outliers_board=gold[f"{case}/outliers_board"] if f"{case}/outliers_board" in gold else None)
     return r_gpu, kw_gpu, r_cpu
 
 
@@ -44,29 +128,17 @@ def check_parity(r_gpu, kw_gpu, r_cpu, tol_b=1e-5, tol_cost=1e-9):
     assert abs(n_gpu - r_cpu["norm2_x"]) <= tol_cost * r_cpu["norm2_x"]
     assert r_gpu["Noutliers_board"] == r_cpu["Noutliers_board"]
     # the solution was written into the caller's arrays, and it is the unpacked b_packed
-    P = r_cpu["problem"]
-    for name, ref_arr in (("intrinsics", P.intrinsics), ("rt_cam_ref", P.rt_cam_ref), ("rt_ref_frame", P.rt_ref_frame),
-                          ("points", P.points), ("calobject_warp", P.calobject_warp)):
+    for name in STATE_ARRAYS:
         if name in kw_gpu and kw_gpu[name] is not None and np.size(kw_gpu[name]):
+            ref_arr = r_cpu["state"][name]
             assert np.allclose(kw_gpu[name], ref_arr, rtol=0, atol=max(tol_b, 1e-5) * max(1., np.abs(ref_arr).max())), name
     if "observations_board" in kw_gpu:
-        assert np.array_equal(kw_gpu["observations_board"][..., 2] < 0, P.observations_board[..., 2] < 0)
+        assert np.array_equal(np.flatnonzero(kw_gpu["observations_board"].reshape(-1, 3)[:, 2] < 0), r_cpu["outliers_board"])
 
 
-@pytest.mark.parametrize("lensmodel,Ncameras,Nframes", [
-    ("LENSMODEL_OPENCV8", 2, 8),
-    ("LENSMODEL_OPENCV4", 3, 6),
-    ("LENSMODEL_PINHOLE", 1, 5),
-    ("LENSMODEL_STEREOGRAPHIC", 2, 5),
-    ("LENSMODEL_CAHVOR", 2, 8),
-    ("LENSMODEL_CAHVORE_linearity=0.37", 2, 8),
-    (SPL3_COVERED, 2, 40),
-    (SPL2_COVERED, 2, 40),
-])
-def test_optimize_matches_cpu_restatement(ref, lensmodel, Ncameras, Nframes):
-    kw, truth = synthetic.make_problem(lensmodel=lensmodel, Ncameras=Ncameras, Nframes=Nframes, W=6, H=5, seed=2,
-                                       pixel_noise=0.2)
-    r_gpu, kw_gpu, r_cpu = run_both(kw)
+@pytest.mark.parametrize("lensmodel,Ncameras,Nframes", RESTATEMENT)
+def test_optimize_matches_cpu_restatement(gold, lensmodel, Ncameras, Nframes):
+    r_gpu, kw_gpu, r_cpu = run_both(gold, f"restatement/{lensmodel}", _restatement(lensmodel, Ncameras, Nframes))
     # Splined solves crawl along weakly-determined knot directions and the reference's stopping rule
     # (squared step < 1e-7) ends them at slightly different points of the same flat valley: the COST
     # agrees to 1e-9 either way, the state only to ~1e-3 there. test_splined_tight_convergence
@@ -81,67 +153,44 @@ def test_optimize_matches_cpu_restatement(ref, lensmodel, Ncameras, Nframes):
 
 
 @pytest.mark.parametrize("lensmodel", [SPL3_COVERED, SPL2_COVERED])
-def test_splined_tight_convergence(ref, lensmodel):
-    from oracle import dogleg_np
-    kw, truth = synthetic.make_problem(lensmodel=lensmodel, Ncameras=2, Nframes=40, W=6, H=5, seed=2, pixel_noise=0.2)
-    tight = dict(update_threshold=1e-24, max_iterations=2000)
-    r_cpu = dogleg_np.optimize(clone(kw), **tight)
+def test_splined_tight_convergence(gold, lensmodel):
+    kw = tight_cases()[lensmodel]
     P = mrcal_b200.Problem(**clone(kw))
-    s = P.optimize(**tight)
+    s = P.optimize(**TIGHT)
     out = P.download(into_inputs=False)
+    b_cpu, norm2_x_cpu = gold[f"tight/{lensmodel}/b_packed"], float(gold[f"tight/{lensmodel}/norm2_x"])
     # both sit at the roundoff floor of the same optimum; the residual state difference is along the
     # flattest knot directions (curvature ~1e-6 of the stiffest), hence 1e-3 rather than 1e-5
-    assert np.abs(out["b_packed"] - r_cpu["b_packed"]).max() <= 1e-3
-    assert abs(s["norm2_x_final"] - r_cpu["norm2_x"]) <= 1e-11 * r_cpu["norm2_x"]
+    assert np.abs(out["b_packed"] - b_cpu).max() <= 1e-3
+    assert abs(s["norm2_x_final"] - norm2_x_cpu) <= 1e-11 * norm2_x_cpu
 
 
-def test_optimize_with_points(ref):
-    kw, truth = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV4", Ncameras=3, Nframes=8, W=6, H=5, seed=4,
-                                       pixel_noise=0.2, Npoints=12, Npoints_fixed=3, which="some")
-    r_gpu, kw_gpu, r_cpu = run_both(kw)
+def test_optimize_with_points(gold):
+    r_gpu, kw_gpu, r_cpu = run_both(gold, "points", _with_points())
     check_parity(r_gpu, kw_gpu, r_cpu)
 
 
-@pytest.mark.parametrize("sel", [
-    dict(do_optimize_intrinsics_core=False, do_optimize_intrinsics_distortions=False, do_optimize_extrinsics=False,
-         do_optimize_frames=True, do_optimize_calobject_warp=False),    # frames only: nothing shared
-    dict(do_optimize_intrinsics_core=True, do_optimize_intrinsics_distortions=True, do_optimize_extrinsics=False,
-         do_optimize_frames=False, do_optimize_calobject_warp=False),   # intrinsics only: nothing eliminated
-    dict(do_optimize_intrinsics_core=False, do_optimize_intrinsics_distortions=False, do_optimize_extrinsics=True,
-         do_optimize_frames=True, do_optimize_calobject_warp=True),
-])
-def test_optimize_selections(ref, sel):
-    kw, truth = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV8", Ncameras=2, Nframes=6, W=6, H=5, seed=5,
-                                       pixel_noise=0.2, perturb=0.3)
-    kw.update(sel)
-    r_gpu, kw_gpu, r_cpu = run_both(kw)
+@pytest.mark.parametrize("sel", SELECTIONS)
+def test_optimize_selections(gold, sel):
+    i = SELECTIONS.index(sel)
+    r_gpu, kw_gpu, r_cpu = run_both(gold, f"selection/{i}", _selection(i))
     check_parity(r_gpu, kw_gpu, r_cpu)
 
 
-@pytest.mark.parametrize("name", ["tri_pinhole_unity_only", "tri_opencv4_boards_points", "tri_stereographic_unity"])
-def test_optimize_with_triangulated_points(ref, name):
+@pytest.mark.parametrize("name", TRIANGULATED)
+def test_optimize_with_triangulated_points(gold, name):
     """Triangulated-point measurements (mrcal.c:5180-5653) in the solve: intrinsics locked, extrinsics free.
     (Rays alone leave the scale of the rig free: something else -- boards, or the unity_cam01 regularization
     -- has to pin it, mrcal.c:5903-5954.)"""
-    kw = clone(dict(problems.golden_cases())[name])
-    kw["do_apply_outlier_rejection"] = False
-    r_gpu, kw_gpu, r_cpu = run_both(kw)
+    r_gpu, kw_gpu, r_cpu = run_both(gold, f"triangulated/{name}", _triangulated(name))
     # (costs here are ~1e-6 rad^2: the absolute stopping rule leaves them less converged in relative terms)
     check_parity(r_gpu, kw_gpu, r_cpu, tol_b=1e-4, tol_cost=1e-6)
     # without outlier rejection markOutliers() never runs and the count stays at its initial 0 (mrcal.c:6416-6417)
     assert r_gpu["Noutliers_triangulated_point"] == 0
 
 
-def test_optimize_outlier_rejection(ref):
-    kw, truth = synthetic.make_problem(lensmodel="LENSMODEL_OPENCV4", Ncameras=2, Nframes=12, W=8, H=7, seed=6,
-                                       pixel_noise=0.3)
-    rng = np.random.default_rng(0)
-    flat = kw["observations_board"].reshape(-1, 3)
-    bad = rng.choice(flat.shape[0], 15, replace=False)
-    flat[bad, :2] += rng.normal(0, 30., (15, 2))          # gross outliers
-    flat[rng.choice(flat.shape[0], 5, replace=False), 2] = -1.   # pre-marked outliers are respected
-    kw["do_apply_outlier_rejection"] = True
-    r_gpu, kw_gpu, r_cpu = run_both(kw)
+def test_optimize_outlier_rejection(gold):
+    r_gpu, kw_gpu, r_cpu = run_both(gold, "outlier_rejection", _outlier_rejection())
     assert r_cpu["passes"] >= 2
     check_parity(r_gpu, kw_gpu, r_cpu)
     assert r_gpu["Noutliers_board"] >= 15

@@ -4,9 +4,9 @@ The error is a small angle computed as th = sqrt(2 - 2 cos) (triangulation.cc:76
 cos (1e-16) is amplified by ~1/th^2 in d th. tests/test_callback_gpu.py compares the triangulated rows of J with
 the compiled reference at 1e-6 instead of the 1e-9 used everywhere else; this file measures why:
 
-  CPU   the reference's own _mrcal_triangulated_error() (oracle/_ref) against a 60-digit evaluation (mpmath) of
-        the same function: the reference's double-precision gradient is itself only good to ~1e-8..1e-7 relative
-        at sub-milliradian angles, far from 1e-9
+  CPU   the reference's own _mrcal_triangulated_error() (oracle/_ref; its values are stored under tests/golden/)
+        against a 60-digit evaluation (mpmath) of the same function: the reference's double-precision gradient
+        is itself only good to ~1e-8..1e-7 relative at sub-milliradian angles, far from 1e-9
   GPU   our device function against the same 60-digit values: at least as close to the truth as the reference is
 
 So a 1e-9 comparison between the two double-precision implementations would be comparing rounding noise."""
@@ -14,6 +14,8 @@ import ctypes as C
 
 import numpy as np
 import pytest
+
+import problems
 
 mp = pytest.importorskip("mpmath")
 
@@ -83,16 +85,14 @@ def _bound(err_true):
     return 200. * EPS / (th * th) + 1e-12
 
 
-def test_reference_gradient_precision(ref, truth):
+def test_reference_gradient_precision(truth):
     cases, tr = truth
-    L = ref.lib()
-    L._mrcal_triangulated_error.restype = C.c_double
+    gold = problems.oracle_golden("precision")
+    assert np.array_equal(gold["cases"], cases)
     worst_grad = 0.
-    for c, (e_true, g_true) in zip(cases, tr):
-        dv1, dt = (C.c_double * 3)(), (C.c_double * 3)()
-        v0, v1, t = (C.c_double * 3)(*c[0:3]), (C.c_double * 3)(*c[3:6]), (C.c_double * 3)(*c[6:9])
-        e = L._mrcal_triangulated_error(dv1, dt, v0, v1, t)
-        eg = _rel(np.array(list(dv1) + list(dt)), g_true)
+    for (e_true, g_true), e_g in zip(tr, gold["error_gradient"]):
+        e = e_g[0]
+        eg = _rel(e_g[1:], g_true)
         assert abs(e - e_true) / e_true <= _bound(e_true)
         assert eg <= _bound(e_true)
         if e_true > 1e-4:           # the residual angles a solve actually sees (0.3 px at f = 1500 is 2e-4 rad)
@@ -103,7 +103,7 @@ def test_reference_gradient_precision(ref, truth):
 
 
 @pytest.mark.gpu
-def test_device_gradient_precision(ref, truth):
+def test_device_gradient_precision(truth):
     from mrcal_b200 import _capi
     cases, tr = truth
     f = _capi.lib.mrcal_b200_debug_triangulated_error
